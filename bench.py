@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on B200: decode tokens/s + RTF, Voxtral-Mini-4B Q4_0, 16 s audio.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--streams B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--streams B] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[4] -- concurrent 16 s streams, B=8 per GPU
@@ -106,6 +106,14 @@ def ensure_gguf(rank: int, barrier):
         synth.write_synthetic_gguf(GGUF_PATH, synth.VoxtralConfig(), seed=SEED_WEIGHTS)
         sys.stderr.write(f"[bench] wrote {GGUF_PATH} in {time.time() - t0:.1f}s\n")
     barrier()
+
+
+def dump_outputs(out_dir: str, **arrays):
+    """Writes each array as out_dir/<name>.npy in float64 (token ids are exact in it), so that the outputs of two
+    builds on the same seeded inputs can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, np.float64))
 
 
 def make_audio(n_streams: int, rank: int) -> np.ndarray:
@@ -329,11 +337,13 @@ def run_ours(args, rank, local_rank, world):
     wall0 = time.perf_counter()
     dec_ms = pre_ms = enc_ms = tot_ms = pf_ms = 0.0
     for _ in range(args.steps):
-        model.transcribe_pcm_dev(dev_audio, B, n, timings=tm)
+        ids = model.transcribe_pcm_dev(dev_audio, B, n, timings=tm)
         dec_ms += tm.decode_ms; pre_ms += tm.preprocess_ms; enc_ms += tm.encode_ms; tot_ms += tm.total_ms
         pf_ms += tm.prefill_ms
     vx.lib().vox_dev_sync(local_rank)
     wall = time.perf_counter() - wall0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, token_ids=ids)
     barrier()
     launches = model.launch_count() - launches0
     K = args.steps
@@ -477,7 +487,13 @@ def main():
     ap.add_argument("--cpu-tokens", type=int, default=6)
     ap.add_argument("--no-streaming", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the token ids of the last timed step (rank 0's streams) to DIR/token_ids.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
     rank, local_rank, world = dist_env()
     if args.impl == "reference":
         run_reference(args, rank, world)

@@ -6,8 +6,9 @@ decode 170-191 (ids < 1000 skipped; id-1000 indexes the vocab *position*; unknow
 skipped; bytes joined then lossy UTF-8), decode_token 194-208.
 
 Pinned: the reference's golden (`[1362,19135,1294,1278,4618,40307,3910,1046]` ->
-" I spoke in the original phonograph.", mod.rs:255-268) needs the real tekken.json,
-which is absent => skip-if-missing; behaviour is otherwise pinned on synthetic vocabularies.
+" I spoke in the original phonograph.", mod.rs:255-268) on the entries of the public Tekken
+vocabulary it uses (tests/golden/tekken_excerpt.json); behaviour is otherwise pinned on
+synthetic vocabularies.
 """
 from __future__ import annotations
 

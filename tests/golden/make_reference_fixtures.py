@@ -1,11 +1,11 @@
-"""Pins the oracle to the REFERENCE'S OWN Python (run in the build container, where /root/reference exists):
+"""Pins the oracle to the REFERENCE'S OWN Python (needs a checkout of the reference repository):
 
-    python tests/golden/make_reference_fixtures.py [--full]
+    python tests/golden/make_reference_fixtures.py <reference checkout>/scripts [--full]
 
 The reference validates its Rust layers against `.npy` files produced by its torch scripts
 (rms_norm.rs:156-211, rope.rs:168-253, swiglu.rs:100-187, conv.rs:113-215, rms_norm.rs:214-291,
 attention.rs:476-619, mel.rs:486-614).  Those scripts are imported here UNMODIFIED from
-/root/reference/scripts and run on our synthetic weights (dequantised to f32, served through a
+the reference's scripts/ directory and run on our synthetic weights (dequantised to f32, served through a
 `get_tensor` shim in place of `safe_open(consolidated.safetensors)`):
 
   A  ref_ops.npz       reference_forward.py  test_rms_norm / test_rope / test_swiglu / test_conv /
@@ -21,9 +21,9 @@ attention.rs:476-619, mel.rs:486-614).  Those scripts are imported here UNMODIFI
                        the GGUF tensor index, so the file is 100 MB and the CPU test stays fast.
   C  ref_chain_full.npz (--full)  the same chain on the full-size seed-42 model (2.5 GB GGUF in /dev/shm).
 
-Stored: inputs, reference outputs (or row subsets + checksums for the big ones).  Consumers:
-tests/test_oracle_vs_reference_py.py (CPU: oracle == reference Python) and tests/test_reference_py_gpu.py
-(-m gpu: CUDA == reference Python).  /root/reference is NOT needed to run those tests.
+Stored: inputs, reference outputs (row subsets of the [positions, dim] activations, plus per-row sums of the conv
+output, audio embeddings and logits, so that each fixture stays below 1 MB).  Consumers: tests/test_oracle_vs_reference_py.py (CPU: oracle == reference Python)
+and tests/test_reference_py_gpu.py (-m gpu: CUDA == reference Python).  The reference is NOT needed to run those tests.
 """
 import ast
 import contextlib
@@ -42,7 +42,7 @@ from oracle import gguf_synth, mel as omel, q4 as oq4  # noqa: E402
 from voxtral_mini_realtime_rs_b200 import synth       # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_SCRIPTS = "/root/reference/scripts"
+REF_SCRIPTS = None       # the reference's scripts/ directory (first command-line argument)
 SEED_FULL = 42
 SEED_SMALL = 11
 AUDIO_SECONDS = 1.0
@@ -156,7 +156,7 @@ def lift_full_forward(cf):
     return ns["lifted_forward"]
 
 
-def make_chain(gguf: gguf_synth.GgufFile, out_name: str, full_rows: bool):
+def make_chain(gguf: gguf_synth.GgufFile, out_name: str, dense: bool):
     gp = load_ref_module("generate_padded_reference.py")
     cf = load_ref_module("compare_full_forward.py")
     audio = omel.peak_normalize(synth.speechlike(AUDIO_SECONDS, seed=AUDIO_SEED))
@@ -188,22 +188,26 @@ def make_chain(gguf: gguf_synth.GgufFile, out_name: str, full_rows: bool):
                logit_row_sums=logits.numpy().astype(np.float64).sum(1),
                emb_row_sums=e.astype(np.float64).sum(1), emb_row_abs_sums=np.abs(e).astype(np.float64).sum(1),
                conv_row_sums=conv.astype(np.float64).sum(1))
-    if full_rows:
-        out.update(audio_embeds=e, hidden=h, conv=conv.astype(np.float32))
+    if dense:       # every conv row, every other embedding / hidden row and the last one
+        rows = np.array(sorted(set(range(0, S4, 2)) | {S4 - 1}), np.int32)
+        crow = np.arange(conv.shape[0], dtype=np.int32)
     else:
         rows = np.array(sorted(set([0, 1, 2, S4 // 2, S4 - 2, S4 - 1])), np.int32)
         crow = np.array(sorted(set([0, 1, conv.shape[0] // 2, conv.shape[0] - 1])), np.int32)
-        out.update(rows=rows, audio_embeds=e[rows], hidden=h[rows], conv_rows=crow, conv=conv[crow].astype(np.float32))
+    out.update(rows=rows, audio_embeds=e[rows], hidden=h[rows], conv_rows=crow, conv=conv[crow].astype(np.float32))
     np.savez_compressed(os.path.join(HERE, out_name), **out)
     marg = (top.values[:, 0] - top.values[:, 1]).numpy()
     print(f"{out_name}: S4={S4} V={V} distinct ids {len(set(r['predicted']))} min top-2 margin {marg.min():.3e}")
 
 
 if __name__ == "__main__":
+    if len(sys.argv) < 2 or not os.path.isdir(sys.argv[1]):
+        sys.exit(__doc__.splitlines()[2])
+    REF_SCRIPTS = sys.argv[1]
     torch.set_num_threads(os.cpu_count() or 8)
     make_ops()
-    make_chain(gguf_synth.GgufFile(synth.build_aliased_gguf_bytes(synth.refshape_config(), SEED_SMALL)), "ref_chain_small.npz", full_rows=True)
+    make_chain(gguf_synth.GgufFile(synth.build_aliased_gguf_bytes(synth.refshape_config(), SEED_SMALL)), "ref_chain_small.npz", dense=True)
     if "--full" in sys.argv:
         if not os.path.exists(FULL_GGUF):
             synth.write_synthetic_gguf(FULL_GGUF, synth.VoxtralConfig(), seed=SEED_FULL)
-        make_chain(gguf_synth.GgufFile(FULL_GGUF), "ref_chain_full.npz", full_rows=False)
+        make_chain(gguf_synth.GgufFile(FULL_GGUF), "ref_chain_full.npz", dense=False)

@@ -1,7 +1,7 @@
-"""oracle/ == the REFERENCE'S OWN torch scripts (CPU; no GPU, no /root/reference needed at run time).
+"""oracle/ == the REFERENCE'S OWN torch scripts (CPU; no GPU, no reference checkout needed at run time).
 
 The fixtures under tests/golden/ref_*.npz were produced by tests/golden/make_reference_fixtures.py, which imports,
-unmodified, /root/reference/scripts/{reference_forward,generate_padded_reference,compare_full_forward}.py -- the scripts
+unmodified, the reference's scripts/{reference_forward,generate_padded_reference,compare_full_forward}.py -- the scripts
 that write the `.npy` files the reference's Rust layer tests load (rms_norm.rs:156-211, rope.rs:168-253,
 swiglu.rs:100-187, conv.rs:113-215, rms_norm.rs:214-291, attention.rs:476-619, mel.rs:486-614) -- and runs them on
 our synthetic weights.  The Rust tests accept 1e-3 (mel: 1e-2) against those files; the oracle is held to 1e-5 per op
@@ -85,7 +85,7 @@ def test_ada_modulation_matches_reference_py(ops, layer0_oracle):  # reference_f
 
 
 # ------------------------------------------------------------------ whole chain
-def _check_chain(om: OracleModel, fx, full_rows: bool, tol_mel, tol_act, tol_logit):
+def _check_chain(om: OracleModel, fx, tol_mel, tol_act, tol_logit):
     audio = omel.peak_normalize(synth.speechlike(float(fx["seconds"]), seed=int(fx["audio_seed"])))
     mel = omel.mel_tensor_from_audio(audio)                      # [1,128,T] via oracle pad + STFT + filterbank
     # generate_padded_reference.py:37-75 (torch.stft + mistral_common mel_filter_bank); mel.rs:534-614 accepts 1e-2
@@ -95,19 +95,15 @@ def _check_chain(om: OracleModel, fx, full_rows: bool, tol_mel, tol_act, tol_log
     cap = {}
     emb = om.encode_audio(fx["mel"][None], cap)
     conv = cap["conv"].numpy()
-    if full_rows:
-        d_conv = maxdiff(conv, fx["conv"])
-        d_emb = maxdiff(emb.numpy(), fx["audio_embeds"])
-    else:
-        d_conv = maxdiff(conv[fx["conv_rows"]], fx["conv"])
-        d_emb = maxdiff(emb.numpy()[fx["rows"]], fx["audio_embeds"])
+    d_conv = maxdiff(conv[fx["conv_rows"]], fx["conv"])
+    d_emb = maxdiff(emb.numpy()[fx["rows"]], fx["audio_embeds"])
     assert d_conv < tol_act, d_conv
     assert maxdiff(conv.astype(np.float64).sum(1), fx["conv_row_sums"]) < 100 * tol_act
     assert d_emb < tol_act, d_emb
     assert maxdiff(emb.numpy().astype(np.float64).sum(1), fx["emb_row_sums"]) < 100 * tol_act
     s4 = emb.shape[0]
     logits, hidden = om.forward_streaming(None, [32] * s4, omel.time_embedding(6.0, 3072), audio_embeds=emb, return_hidden=True)
-    h = hidden.numpy() if full_rows else hidden.numpy()[fx["rows"]]
+    h = hidden.numpy()[fx["rows"]]
     d_h = maxdiff(h, fx["hidden"])
     assert d_h < tol_act * 5, d_h
     lg = logits.numpy()
@@ -129,14 +125,15 @@ def test_chain_small_matches_reference_py():
     (compare_full_forward.py:262-361) on the reference-shaped small model."""
     fx = np.load(os.path.join(GOLD, "ref_chain_small.npz"))
     om = OracleModel(gguf_synth.GgufFile(synth.build_aliased_gguf_bytes(synth.refshape_config(), seed=11)))
-    r = _check_chain(om, fx, True, tol_mel=2e-4, tol_act=2e-4, tol_logit=1e-3)
+    r = _check_chain(om, fx, tol_mel=2e-4, tol_act=2e-4, tol_logit=1e-3)
     print("oracle vs reference python (small):", r)
 
 
 @pytest.mark.slow
-@pytest.mark.skipif(not os.path.exists(FULL_GGUF), reason="full-size synthetic GGUF not generated (tests/test_golden_gpu.py does it on the GPU box)")
 def test_chain_full_matches_reference_py():
     fx = np.load(os.path.join(GOLD, "ref_chain_full.npz"))
+    if not os.path.exists(FULL_GGUF):
+        synth.write_synthetic_gguf(FULL_GGUF, synth.VoxtralConfig(), seed=42)
     om = OracleModel(FULL_GGUF)
-    r = _check_chain(om, fx, False, tol_mel=2e-4, tol_act=2e-4, tol_logit=1e-3)
+    r = _check_chain(om, fx, tol_mel=2e-4, tol_act=2e-4, tol_logit=1e-3)
     print("oracle vs reference python (full):", r)

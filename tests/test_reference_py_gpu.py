@@ -1,5 +1,5 @@
 """CUDA path == the REFERENCE'S OWN torch scripts (fixtures tests/golden/ref_*.npz, generator
-tests/golden/make_reference_fixtures.py: /root/reference/scripts/{reference_forward,generate_padded_reference,
+tests/golden/make_reference_fixtures.py: the reference's scripts/{reference_forward,generate_padded_reference,
 compare_full_forward}.py run unmodified on our synthetic weights).  Everything through the C ABI.
 
 Bounds: north_star -- encoder hidden states / audio embeddings within 1e-3 abs; logits of O(1) within 2e-3
@@ -24,7 +24,7 @@ def maxdiff(a, b):
     return float(np.abs(np.asarray(a, np.float64) - np.asarray(b, np.float64)).max())
 
 
-def _check_chain(vx, model, fx, full_rows, what):
+def _check_chain(vx, model, fx, what):
     audio = synth.speechlike(float(fx["seconds"]), seed=int(fx["audio_seed"]))
     # --- mel: peak-normalise + pad + GPU STFT/filterbank vs torch.stft + mistral_common filterbank
     ms = vx.MelSpectrogram.voxtral(0)
@@ -39,10 +39,7 @@ def _check_chain(vx, model, fx, full_rows, what):
         conv = model.debug("conv").reshape(-1, model.info["enc_dim"])
     finally:
         model.debug("capture_off")
-    if full_rows:
-        d_conv, d_emb = maxdiff(conv, fx["conv"]), maxdiff(emb, fx["audio_embeds"])
-    else:
-        d_conv, d_emb = maxdiff(conv[fx["conv_rows"]], fx["conv"]), maxdiff(emb[fx["rows"]], fx["audio_embeds"])
+    d_conv, d_emb = maxdiff(conv[fx["conv_rows"]], fx["conv"]), maxdiff(emb[fx["rows"]], fx["audio_embeds"])
     assert d_conv < 1e-3, d_conv
     assert d_emb < 1e-3, d_emb
     assert maxdiff(emb.astype(np.float64).sum(1), fx["emb_row_sums"]) < 2e-2
@@ -69,7 +66,7 @@ def test_chain_small_vs_reference_py(vx):
     data = synth.build_aliased_gguf_bytes(synth.refshape_config(), seed=11)
     model = vx.Q4ModelLoader.from_bytes(data).load(0, max_batch=1, max_mel_frames=1000)
     try:
-        _check_chain(vx, model, fx, True, "reference-shaped small model")
+        _check_chain(vx, model, fx, "reference-shaped small model")
     finally:
         model.close()
 
@@ -81,7 +78,7 @@ def test_chain_full_vs_reference_py(vx):
         synth.write_synthetic_gguf(FULL_GGUF, synth.VoxtralConfig(), seed=42)
     model = vx.Q4ModelLoader.from_file(FULL_GGUF).load(0, max_batch=1, max_mel_frames=1000)
     try:
-        _check_chain(vx, model, fx, False, "full-size seed-42 model")
+        _check_chain(vx, model, fx, "full-size seed-42 model")
     finally:
         model.close()
 
